@@ -11,6 +11,12 @@ the elapsed time, sum of the counters) closes the run.
 
 Prints ONE JSON line (rank 0).  Timing: CUDA events on the launching stream around each step kernel, L2 flushed
 between steps (a 256 MiB write, outside the events), max over ranks.
+
+  --dump-outputs DIR   rank 0 writes what the timed path returned after its last timed step as DIR/<name>.npy (float64):
+                       <part>_q, <part>_v (+ <part>_jq, <part>_jqd) of the stepped paths, z / status / pivots of --workload lcp.
+                       Inputs come from fixed seeds, so two builds run with the same arguments can be compared file by file.
+                       Compare dumps of the same arm: --impl reference steps its own, smaller seeded batch (the workload's
+                       ref_sample envs), so its files have other shapes and other envs than those of the CUDA arm.
 """
 import argparse
 import json
@@ -26,6 +32,9 @@ import numpy as np
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path[:0] = [ROOT]
+sys.dont_write_bytecode = True       # modules that building does not import (tests/oracle_api.py, moby_b200/lcp.py, ...) leave no
+                                     # __pycache__ in the source tree: the benchmark writes nothing there
+DUMP_BYTES = 60_000_000              # --dump-outputs: above this the dump is a seeded sample of the envs (under 64 MB in all)
 
 # Workloads = BASELINE.json configs.  "small" (configs[1]) is the one the metric is quoted on and the default; the
 # others are the larger single-GPU configurations, selectable with --workload.
@@ -168,6 +177,32 @@ class ClockSampler:
                 if val.lower().startswith("active"):
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def _dump_outputs(out_dir, parts):
+    """--dump-outputs: parts = [(prefix, axis, {name: array})], `axis` the env (or problem) index of every array of the part.
+    Writes out_dir/<prefix><name>.npy in float64.  When everything would exceed DUMP_BYTES, each part keeps the same fixed,
+    seeded sample of its envs in every array, and the sampled indices go to out_dir/<prefix>sample.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n_of = lambda axis, arrs: next(iter(arrs.values())).shape[axis]      # noqa: E731
+    total = 8 * sum(sum(a.size for a in arrs.values()) + n_of(axis, arrs) for _, axis, arrs in parts)   # arrays + sample indices
+    frac = min(1.0, DUMP_BYTES / total)
+    for prefix, axis, arrs in parts:
+        if frac < 1.0:
+            n = n_of(axis, arrs)
+            idx = np.sort(np.random.default_rng(0).choice(n, int(n * frac), replace=False))
+            np.save(os.path.join(out_dir, prefix + "sample.npy"), idx.astype(np.float64))
+            arrs = {k: np.take(a, idx, axis=axis) for k, a in arrs.items()}
+        for k, a in arrs.items():
+            np.save(os.path.join(out_dir, prefix + k + ".npy"), np.asarray(a, np.float64))
+
+
+def _state_arrays(state, joints):
+    """{q, v[, jq, jqd]} of one batch: state = (q, v) [body][7|6][env], joints = (jq, jqd) [dof][env] or None."""
+    out = dict(zip(("q", "v"), state))
+    if joints is not None:
+        out.update(zip(("jq", "jqd"), joints))
+    return out
 
 
 def _cpu_baseline(scene, q, v, joints, dt, n_envs, n_steps, threads):
@@ -375,6 +410,12 @@ def run_reference(args, rank, world):
     for _ in range(args.steps):
         c1 = [b.run(DT, 1, threads=cores) for b in batches]
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        parts = []
+        for nm, b in zip(names, batches):
+            joints = None if b.rc is None else [np.stack(x, axis=1) for x in zip(*(b.get_joint_state(i) for i in range(b.e1 - b.e0)))]
+            parts.append((nm + "_", -1, _state_arrays(b.get_state_soa(), joints)))
+        _dump_outputs(args.dump_outputs, parts)
     val = sample * args.steps / el
     c0 = {"lcp_solves": sum(c["lcp_solves"] for c in c0)}
     c1 = {"lcp_solves": sum(c["lcp_solves"] for c in c1)}
@@ -443,6 +484,8 @@ def run_lcp(args, rank, world, local_rank):
     t_dev = sum(a.elapsed_time(b) for a, b in ev) * 1e-3
     ok = int(((status == 0) | (status == 1)).sum().item())
     piv_mean = float(pivots.double().mean().item())
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(args.dump_outputs, [("", 0, {"z": z.cpu().numpy(), "status": status.cpu().numpy(), "pivots": pivots.cpu().numpy()})])
     # end to end with host buffers through the host-form entry point (H2D M, q; solve; D2H z inside the call)
     Mh, qh = M.cpu().numpy(), q.cpu().numpy()
     nb_e2e = min(batch, 32768)
@@ -508,6 +551,7 @@ def main():
     ap.add_argument("--min-step", default="scene", choices=["scene", "default"],
                     help="scene: min-step-size of the source scenes (test/box.xml: 1e-3, bouncing-ball.xml: sqrt(eps)); "
                          "default: sqrt(eps) everywhere (TimeSteppingSimulator.cpp:48)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -585,6 +629,9 @@ def main():
     barrier()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:           # before the profile pass below steps the same batches further
+        _dump_outputs(args.dump_outputs, [(nm + "_", -1, _state_arrays(ps.get_state(), ps.get_joint_state() if sc.rc is not None else None))
+                                          for nm, ps, sc in zip(names, part_sims, part_scenes)])
     kernel_ms = [a.elapsed_time(b) for a, b in ev]
     t_dev = sum(kernel_ms) * 1e-3
     cnt = sim.counters()

@@ -1,11 +1,14 @@
 """Sub-samples the reference's golden trajectories (regress/*.dat, written by programs/regress.cpp:78-95:
 `t q0 q1 ...` per step, generalized Euler coordinates of every body) into small fixtures.
-Run in the build container only (needs /root/reference); the fixtures are committed.
+Needs the original Moby sources: MOBY_SOURCE_DIR names a Moby checkout.  The fixtures are committed.
 """
 import os
+import sys
 import numpy as np
 
-REF = "/root/reference/regress"
+if not os.environ.get("MOBY_SOURCE_DIR"):
+    sys.exit("set MOBY_SOURCE_DIR to a checkout of the original Moby sources (this script reads its regress/*.dat)")
+REF = os.path.join(os.environ["MOBY_SOURCE_DIR"], "regress")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 

@@ -13,6 +13,7 @@ import os
 import numpy as np
 import pytest
 
+import moby_sources
 from moby_b200 import scenes
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -64,11 +65,10 @@ def test_device_code_matches_oracle_on_the_pendulum(oracle, hostsim):
     assert hf.counters_dict()["lcp_solves"] == c["lcp_solves"] and hf.counters_dict()["contacts"] == c["contacts"]
 
 
+@moby_sources.needed
 def test_xml_pendulum_scene_loads_like_the_builder():
     from moby_b200 import xml_scene
-    path = "/root/reference/example/contact-constrained-pendulum/contact-constrained-pendulum.xml"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
+    path = os.path.join(moby_sources.EXAMPLE, "contact-constrained-pendulum", "contact-constrained-pendulum.xml")
     s, info = xml_scene.load_xml(path, n_envs=1)
     b = scenes.contact_constrained_pendulum(1)
     assert info["bodies"] == {"l1": 0, "world": 1}

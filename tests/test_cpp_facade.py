@@ -6,6 +6,8 @@ import subprocess
 import numpy as np
 import pytest
 
+import moby_sources
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CPP = os.path.join(ROOT, "tests", "cpp")
 
@@ -52,7 +54,7 @@ def test_facade_sitting_box_matches_oracle(sitting_box, oracle):
 
 
 # ---- Moby::XMLReader::read of the facade (include/b200moby_xml.hpp) against the Python loader ----
-REF = "/root/reference/example"
+REF = moby_sources.EXAMPLE
 
 
 def _dump(sitting_box, path):
@@ -96,7 +98,7 @@ def _check_against_python_loader(sitting_box, path):
                 assert s.NK[a * nb + b, 0] == 4 and s.mu_coulomb[a * nb + b, 0] == 0.0 and s.epsilon[a * nb + b, 0] == 0.0
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+@moby_sources.needed
 @pytest.mark.parametrize("rel", ["simple-contact/simplest.xml", "bouncing-ball/bouncing-ball.xml", "stacks/sphere-stack.xml", "stacks/stack.xml",
                                  "rimless-wheel/wheel.xml", "contact-constrained-pendulum/contact-constrained-pendulum.xml"])
 def test_cpp_xml_reader_loads_reference_scenes(sitting_box, rel):

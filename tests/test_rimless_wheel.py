@@ -19,6 +19,7 @@ import os
 import numpy as np
 import pytest
 
+import moby_sources
 from moby_b200 import scenes
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -96,11 +97,10 @@ def test_device_code_matches_oracle_on_wheels(oracle, hostsim, stab):
     assert (q[1, 0, :] > 0.5).all()          # every wheel rolled past its first spoke
 
 
+@moby_sources.needed
 def test_xml_wheel_scene_loads_like_the_builder():
     from moby_b200 import xml_scene
-    path = "/root/reference/example/rimless-wheel/wheel.xml"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
+    path = os.path.join(moby_sources.EXAMPLE, "rimless-wheel", "wheel.xml")
     s, info = xml_scene.load_xml(path, n_envs=1)
     assert info["bodies"] == {"GROUND": 0, "WHEEL": 1}
     b = scenes.rimless_wheel(1, theta_dot=0.0)

@@ -5,12 +5,13 @@ import os
 import numpy as np
 import pytest
 
+import moby_sources
 from moby_b200 import scenes, sdf_scene
 
-SDF = "/root/reference/example/ur10/model.sdf"
+SDF = os.path.join(moby_sources.EXAMPLE, "ur10", "model.sdf")
 
 
-@pytest.mark.skipif(not os.path.exists(SDF), reason="reference tree not present (GPU box)")
+@moby_sources.needed
 def test_ur10_sdf_matches_the_transcribed_tables():
     name, links, joints = sdf_scene.load_sdf_model(SDF)
     assert name == "ur10_schunk_hybrid" and len(links) == len(scenes._UR10_LINKS) == 10

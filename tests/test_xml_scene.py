@@ -1,14 +1,13 @@
 """Moby XML scene loader (moby_b200/xml_scene.py): the reference's own example files load into the same batch
 descriptors as the hand-written scene builders, and an inline scene steps on the oracle."""
-import os
-
 import numpy as np
 import pytest
 
+import moby_sources
 from moby_b200 import scenes, xml_scene
 
-REF = "/root/reference/example"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+REF = moby_sources.EXAMPLE
+needs_ref = moby_sources.needed
 
 INLINE = """
 <XML>
