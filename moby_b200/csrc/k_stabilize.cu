@@ -25,7 +25,13 @@ __device__ __forceinline__ void stabilize_env(const G& g, const SimParams& P, in
 // Two launches per step.  mode 0 (select): every env evaluates its pairwise distances once and, if some pair is closer than
 // eps, puts itself on `queue`.  mode 1 (process): the queued envs are stabilized, 32 per warp.  With one launch over all
 // envs a warp of 32 consecutive envs holds on average five that need the LCP and the line search (17 % of configs[1]) and
-// runs as long as the slowest of them: compaction cuts the warps that walk the expensive path sixfold (2.2 -> ~1 ms per step).
+// runs as long as the slowest of them: compaction cuts the warps that walk the expensive path sixfold.
+// The queue's length is known on the device only (the step is one captured graph), so the process launch is a full
+// resident grid (sim_kernels.cu) and deals warp ranks round the blocks first: a short queue (4,400 of 65,536 envs on
+// configs[1]) still reaches every SM, about one warp each.  Packed block by block it filled 38 blocks on 38 of 148 SMs
+// (1.94 ms per step on a B200).  Measured with that layout and fewer envs per warp: 32 / 16 / 8 / 4 lanes -> 1.46 / 1.51 /
+// 1.58 / 1.85 ms.  The pass is bound by the latency of its dependent local-memory chains, and local memory is interleaved
+// across a warp's lanes: a partly filled warp moves the same sectors for fewer envs, and more warps per SM share the L1.
 template <int ND, int NI>
 __global__ void __launch_bounds__(128) stabilize_thread_kernel(SimParams P, int mode, int* queue, int* count) {
   double wd[ND];
@@ -46,7 +52,8 @@ __global__ void __launch_bounds__(128) stabilize_thread_kernel(SimParams P, int 
     return;
   }
   const int n = queue ? *count : P.n_envs;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) { stabilize_env(g, P, queue ? queue[i] : i, m, s, lc); envs++; }
+  const int first = (((threadIdx.x >> 5) * gridDim.x + blockIdx.x) << 5) + (threadIdx.x & 31);
+  for (int i = first; i < n; i += gridDim.x * blockDim.x) { stabilize_env(g, P, queue ? queue[i] : i, m, s, lc); envs++; }
   for (int k = 0; k < CNT_COUNT; k++) {
     unsigned long long v = lc[k];
     for (int o = 16; o > 0; o >>= 1) { const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o); v = (k == CNT_MAX_N) ? (u > v ? u : v) : v + u; }

@@ -64,6 +64,7 @@ struct b200moby_sim {
   bool any_thread_class = false;
   // constraint stabilization phase (k_stabilize.cu): thread-per-env variant, or -1 = warp per env over `stab_scratch`
   int stab_variant = -1, stab_grid = 1; double* stab_scratch = nullptr; size_t stab_stride = 0, stab_nd_env = 0, stab_nd_all = 0;
+  int stab_proc_grid = 1;    // thread-per-env process launch: every block that can be resident at once
   bool fused = false;        // B200MOBY_FUSED=1: the single fused warp-per-env kernel (kept for comparison)
   long long launches = 0;
   // the impact classes of one round touch disjoint envs: they run on side streams so that the tail of one class
@@ -371,6 +372,12 @@ b200moby_status plan_launch(b200moby_sim* h) {
       B2M_CUDA(cudaMalloc((void**)&h->stab_scratch, h->stab_stride * (size_t)h->stab_grid * 4 * sizeof(double)));
       h->allocs.push_back(h->stab_scratch);
     }
+    if (h->stab_variant >= 0) {
+      int per_sm = 0;
+      B2M_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, b2m_k_stabilize_thread(h->stab_variant), 128, 0));
+      if (per_sm < 1) return b2m_fail(B200MOBY_ERR_UNSUPPORTED, "stabilization kernel does not fit an SM");
+      h->stab_proc_grid = sms * per_sm;
+    }
     if (h->stab_variant >= 0 && env_int("B200MOBY_STAB_SELECT", 1) != 0) {
       b200moby_status s4;
       if ((s4 = dev_zero(h, (size_t)ne + 1, &h->stab_queue)) != B200MOBY_OK) return s4;
@@ -448,7 +455,7 @@ b200moby_status launch_stabilize(b200moby_sim* h, cudaStream_t s) {
       return timed_launch(h, 4 + ncls, b2m_k_stabilize_warp(), dim3(h->stab_grid), dim3(128), aw, 0, s);
     }
     void* a[] = {&Ps, &mode, &queue, &count};
-    return timed_launch(h, 4 + ncls, b2m_k_stabilize_thread(h->stab_variant), dim3(blocks), dim3(128), a, 0, s);
+    return timed_launch(h, 4 + ncls, b2m_k_stabilize_thread(h->stab_variant), dim3(h->stab_proc_grid), dim3(128), a, 0, s);
   }
   Ps.gscratch = h->stab_scratch; Ps.gstride = h->stab_stride;
   int* queue = nullptr; int* count = nullptr;
