@@ -8,7 +8,8 @@
 // one-thread group, the class's working set in the thread's local memory (interleaved by the hardware, so equal indices
 // of neighbouring envs coalesce).  Divergence is bounded by a small per-env budget of solver iterations: an env that
 // needs more is abandoned untouched and re-run by the straggler kernel (many threads per env, shortest latency per
-// pivot), and from then on its recorded cost sends it to the hard queue directly (SimParams::cost).
+// pivot), and from then on its recorded cost sends it to the hard queue directly (SimParams::cost).  An env whose first
+// lcp_fast rung does not verify is handed on the same way (EnvCtx::first_rung), without that cost.
 // Same arithmetic per env as the warp and block kernels: results are bit-identical.
 #include "sim_kernel_util.cuh"
 using namespace b2m;
@@ -33,7 +34,7 @@ __global__ void __launch_bounds__(128) impact_thread_kernel(SimParams P, double 
   const int lane = threadIdx.x & 31, warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
   for (int i = warp * lanes + lane; lane < lanes && i < count; i += nwarps * lanes) {
     for (int k = 0; k < CNT_COUNT; k++) lc[k] = 0;
-    EnvCtx cx; cx.limit = P.pivot_budget > 0; cx.budget = P.pivot_budget;
+    EnvCtx cx; cx.limit = P.pivot_budget > 0; cx.budget = P.pivot_budget; cx.first_rung = P.first_rung_handoff != 0;
     if (env_impact(g, P, q_at(P, round, slot, i), m, dt, round, lc, cx)) add_counters(tot, lc);
     envs++;                                            // envs handed to this launch (deferred ones included), like the warp kernel
   }

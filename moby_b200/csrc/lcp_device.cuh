@@ -1084,10 +1084,11 @@ B2M_DEV inline double pow10i(int e) {
 
 // lcp_fast_regularized (LCP.cpp:212-350).  stats[0] += lcp_fast calls, stats[1] += pivots as the
 // reference counts them, stats[2] += iterations actually executed (thread 0 only, may be NULL).
+// defer_unverified: return LCP_DEFER instead of climbing the regularisation rungs when the first solve does not verify.
 template <class G>
 B2M_DEV int lcp_fast_regularized(const G& g, int n, const double* M, int ldm, const double* q, double zero_tol, bool warm,
                                     int min_exp, int step_exp, int max_exp, double* z, double* wd, int* wi,
-                                    int* pivots_out, long long* stats, int* budget = nullptr) {
+                                    int* pivots_out, long long* stats, int* budget = nullptr, bool defer_unverified = false) {
   if (n == 0) { if (pivots_out) *pivots_out = 0; return LCP_OK; }
   const double offdiag = norm_inf_offdiag(g, n, M, ldm);
   const double ZERO_TOL = (zero_tol > 0.0) ? zero_tol : n * norm_inf_with(g, n, M, ldm, 0.0, offdiag) * B2M_NEAR_ZERO;   // :228
@@ -1102,6 +1103,7 @@ B2M_DEV int lcp_fast_regularized(const G& g, int n, const double* M, int ldm, co
     if (pivots_out) *pivots_out = piv;   // reference leaves `pivots` at the last solve's count here (:252-255)
     return st;
   }
+  if (defer_unverified) return LCP_DEFER;
   int attempt = 0;
   for (int rf = min_exp; rf < max_exp; rf += step_exp, attempt++) {                 // :281-340
     const double lambda = pow10i(rf);

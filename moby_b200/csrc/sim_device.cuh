@@ -84,6 +84,7 @@ struct SimParams {
   int* qctl;                   // [2][B2M_ROUNDS_MAX][B2M_SLOTS + 1] counts, then heads (slot B2M_SLOTS: the advance launch's own head)
   int n_classes; int class_nmax[B2M_MAX_CLASSES]; int class_cmax[B2M_MAX_CLASSES];
   int class_budget[B2M_MAX_CLASSES];   // solver-iteration budget of the class's thread-per-env launch (0: none); an env whose cost history reaches it goes to the hard queue instead
+  int first_rung_handoff;      // != 0: the thread-per-env classes hand on an env whose first lcp_fast rung does not verify (EnvCtx)
   // debug taps (may be null)
   double* tap_MM; double* tap_qq; double* tap_z; int* tap_n;
   // reduced-coordinate articulated body (null / 0 when the scene has none)
@@ -193,7 +194,14 @@ enum { S_NPAIRS = 0, S_NCON = 1, S_NC = 2, S_NGC = 3, S_N = 4, S_NISL = 5, S_FLA
 // Per-env solver budget: when `limit` is set and an env's pivots in this launch exceed it, the env's step is
 // abandoned without touching its stored state and the env is queued for the block-per-env kernel, which redoes the
 // step with many more threads per pivot (same arithmetic, same results).  Keeps one hard LCP from holding a whole SM.
-struct EnvCtx { int budget; bool limit; void* ladder = nullptr; };   // ladder: LadderCtx of an impact_warp_kernel warp (the rungs of the Lemke ladder become tasks other warps take, lcp_device.cuh)
+// first_rung: a one-thread group under a budget (the thread-per-env classes) also hands its env on as soon as the first
+// rung of the lcp_fast ladder does not verify.  Such an env has three more rungs and maybe the Lemke ladder ahead, work
+// that holds up the 31 other envs of its warp; the hard-queue launch running next to the classes takes it at once.
+struct EnvCtx {
+  int budget; bool limit;
+  void* ladder = nullptr;      // LadderCtx of an impact_warp_kernel warp (the rungs of the Lemke ladder become tasks other warps take, lcp_device.cuh)
+  bool first_rung = true;
+};
 
 // per-env solver statistics (SimParams::env_stat): the counters an env added to `lc` since `base` was taken
 struct EnvStatBase { unsigned long long fail, lemke, fast, solves, pivots; };
@@ -1454,7 +1462,7 @@ B2M_DEV B2M_NOINL bool solve_qp(const G& g, const SimParams& P, int e, EnvMem& m
 #define B2M_STAMP(row) do {} while (0)
 #endif
   B2M_STAMP(PH_CONTACTS);                                                            // timeline mode: before the lcp_fast ladder
-  { B2M_PROF_T0(m); st = lcp_fast_regularized(g, n, m.MM, n, m.qq, -1.0, true, -20, 4, -8, m.z, m.work, m.iwork, &piv, stats, bud); B2M_PROF_ADD(m, g, PH_FAST); }   // :219
+  { B2M_PROF_T0(m); st = lcp_fast_regularized(g, n, m.MM, n, m.qq, -1.0, true, -20, 4, -8, m.z, m.work, m.iwork, &piv, stats, bud, G::size == 1 && cx.limit && cx.first_rung); B2M_PROF_ADD(m, g, PH_FAST); }   // :219
   B2M_STAMP(PH_PROBLEM);                                                             // after it
   if (st == LCP_DEFER) return false;
   long long fast_calls = stats[0], pivots = stats[1], executed = stats[2], lemke_calls = 0;
@@ -2017,7 +2025,9 @@ B2M_DEV bool env_impact(const G& g, const SimParams& P, int e, EnvMem& m, double
   B2M_PROF_ADD(m, g, PH_CONTACTS); }
   lc[CNT_CONTACTS] = c0; lc[CNT_OVERFLOW] = o0;                  // counted by the advance phase
   if (!process_constraints(g, P, e, m, lc, cx)) {
-    if (g.tid == 0) { const int hc = P.pivot_budget > P.hard_cost ? P.pivot_budget : P.hard_cost; q_push(P, round, B2M_SLOT_STRAGGLER, e); if (P.cost && P.cost[e] < 4 * hc) P.cost[e] = 4 * hc; }
+    // only an env that ran out of its budget is marked expensive: one handed on after its first lcp_fast rung keeps its cost
+    // history (marked, ~1,400 such envs per step of configs[1] would sit in the hard queue for several steps and lengthen it)
+    if (g.tid == 0) { const int hc = P.pivot_budget > P.hard_cost ? P.pivot_budget : P.hard_cost; q_push(P, round, B2M_SLOT_STRAGGLER, e); if (P.cost && cx.budget < 0 && P.cost[e] < 4 * hc) P.cost[e] = 4 * hc; }
     g.sync();
     return false;
   }
